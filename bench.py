@@ -7,6 +7,7 @@ Headline (default, `--config cfg2`): `MulticlassConfusionMatrix(num_classes=1000
     python bench.py --gpus N --steps K --warmup W            # ours (N>1: launched by torchrun, one rank per GPU)
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU implementation on the host cores
     python bench.py --config cfg3|cfg4|cfg5 [...]            # the other BASELINE.json configs, same line format
+    python bench.py --steps K --warmup W --dump-outputs DIR  # + DIR/confmat.npy: what the last timed step computed
 
 Prints ONE JSON line (rank 0).  See DESIGN.md §4 for how each field is obtained.  The default cfg2 line also carries
   config.sync   the cross-rank state sync of the [C, C] confusion matrix, timed on its own (N > 1)
@@ -443,6 +444,7 @@ def run_ours(args) -> dict:
     # update, weighted by how often the batch was cycled through; the expectations are combined over ranks by a DIFFERENT path
     # than the one under test (all_gather + local sum instead of the metric's all-reduce)
     expect = torch.zeros(N_CLASSES, N_CLASSES, dtype=torch.long, device=dev)
+    last_batch = (args.steps - 1) % N_ROT
     for b in range(N_ROT):
         times_used = uses[b] + len(range(b, args.steps, N_ROT))  # spin-up + the K timed steps
         if times_used == 0:
@@ -451,6 +453,8 @@ def run_ours(args) -> dict:
         single.update(*dev_batches[b])
         torch.cuda.synchronize(dev)
         expect += single.confmat * times_used
+        if b == last_batch:
+            last_step = single.compute().clone()
     if distributed:
         slab = torch.empty((world, N_CLASSES, N_CLASSES), dtype=torch.long, device=dev)
         dist.all_gather_into_tensor(slab, expect)
@@ -460,6 +464,17 @@ def run_ours(args) -> dict:
         dist.all_reduce(n_updates)  # ranks spin for the same wall time, not the same number of updates
     assert int(result.sum()) == N_ROWS * int(n_updates), "confusion matrix lost samples"
     assert torch.equal(result, expect), "timed + synced confusion matrix differs from the sum of isolated per-batch updates"
+    if args.dump_outputs:
+        # The timed state also holds the spin-up updates, whose number depends on wall time; what the LAST timed step adds
+        # is the confusion matrix of its batch alone (the check above ties these isolated matrices to the timed state), which
+        # is the same from run to run.  Over N ranks: the sum of every rank's last step, as compute() would return it.
+        if distributed:
+            dist.all_reduce(last_step)
+        if rank == 0:
+            import numpy as np
+
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "confmat.npy"), last_step.cpu().numpy().astype(np.float64))
 
     per_rank_ms = [ms_updates / args.steps]
     if distributed:  # every rank's own window, for the record (the value uses the maximum)
@@ -618,7 +633,13 @@ def main() -> None:
     ap.add_argument("--config", default="cfg2", choices=["cfg2", "cfg3", "cfg4", "cfg5"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the cfg5 leg and the ATen-on-GPU arm of the cfg2 line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the [C, C] confusion matrix of the last timed step as DIR/confmat.npy (float64; cfg2, --impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config != "cfg2"):
+        ap.error("--dump-outputs covers the cfg2 line of --impl ours")
     # stdout carries exactly ONE JSON line: everything else that writes to file descriptor 1 (NCCL's version banner with
     # NCCL_DEBUG=VERSION, library chatter) is diverted to stderr; the JSON goes to a private duplicate of the real stdout
     sys.stdout.flush()

@@ -37,6 +37,9 @@ def build(verbose: bool = False) -> str:
         name="metrics_b200_torch_ops",
         sources=[os.path.join(_HERE, "csrc", "torch_ops", "ops.cpp")],
         extra_cflags=["-O2", "-std=c++17"],
+        # no .cu source here, but with_cuda makes cpp_extension derive nvcc arch flags, which fails on a machine without a
+        # GPU unless TORCH_CUDA_ARCH_LIST is set; an explicit arch skips that probe
+        extra_cuda_cflags=["-gencode=arch=compute_100a,code=sm_100a"],
         extra_include_paths=[os.path.join(cpp_extension.CUDA_HOME or "/usr/local/cuda", "include")],
         extra_ldflags=[f"-L{lib_dir}", "-lmetrics_b200", "-Wl,-rpath,'$$ORIGIN/..'", "-lc10_cuda", "-ltorch_cuda"],
         build_directory=_BUILD_DIR,
